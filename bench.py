@@ -1,8 +1,9 @@
 #!/usr/bin/env python
-"""Benchmark of the Swapping-Autoencoder training hot path on B200 (contract: see the task brief / DESIGN.md §7).
+"""Benchmark of the Swapping-Autoencoder training hot path on B200 (DESIGN.md §7).
 
   python bench.py --gpus N --steps K --warmup W            # our arm (one process per GPU under torchrun for N > 1)
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU (native-PyTorch) path = oracle port
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/*.npy
 
 A "step" is one ``train_one_step`` call — a discriminator OR a generator half-step over one batch, exactly the unit
 the reference's own iteration counter advances by (reference util/iter_counter.py:54, SURVEY.md §8(d)); lazy R1
@@ -283,6 +284,25 @@ def r1_position(d_steps, every):
     return (best[1] if best else 0), target
 
 
+DUMP_SAMPLE = 4096
+
+
+def dump_outputs(out_dir, losses, named_params):
+    """Writes what the last timed half-step hands its caller — its losses (``loss.<name>.npy``, float64) and the parameters
+    it leaves behind (``param.<name>.npy``, float32; tensors above DUMP_SAMPLE elements at DUMP_SAMPLE indices drawn from a
+    fixed seed: 1.6 MB in all for the default nets) — so that two builds can be compared output for output on identical inputs.
+    The inputs are seeded and the kernels reduce in a fixed order, so repeated runs of one build write the same values."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in losses.items():
+        np.save(os.path.join(out_dir, "loss.%s.npy" % k), np.asarray(float(v), dtype=np.float64))
+    for name, p in named_params:
+        flat = p.detach().float().reshape(-1).cpu().numpy()
+        if flat.size > DUMP_SAMPLE:
+            flat = flat[np.sort(np.random.RandomState(0).choice(flat.size, DUMP_SAMPLE, replace=False))]
+        np.save(os.path.join(out_dir, "param.%s.npy" % name), flat)
+
+
 def run_ours(args, rank, world, local):
     import swapping_autoencoder_pytorch_b200 as S
     from swapping_autoencoder_pytorch_b200 import _lib, backend
@@ -348,7 +368,7 @@ def run_ours(args, rank, world, local):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
         return {"ms": ms, "launches": launches, "clocks": clocks, "r1": kinds.count("D+R1"), "phases": phases,
-                "per_kind_ms": {kd: sum(v) / len(v) for kd, v in per_kind.items()}}
+                "per_kind_ms": {kd: sum(v) / len(v) for kd, v in per_kind.items()}, "last_losses": out}
 
     def warm(resident):
         # at least 4 untimed half-steps: D, G, D, G — both step kinds twice, so the caching allocator and every kernel
@@ -378,6 +398,9 @@ def run_ours(args, rank, world, local):
 
     host, resident, n_warm, dev, e2e = measure(PER_GPU_BATCH, True)
     images = args.steps * PER_GPU_BATCH * world
+    if args.dump_outputs and rank == 0:
+        # the e2e loop ran last: its final half-step is the last timed step
+        dump_outputs(args.dump_outputs, e2e["last_losses"], model.singlegpu_model.named_parameters())
 
     strong = None
     if world > 1 and 32 % world == 0 and (32 // world) % 2 == 0 and not args.no_strong:
@@ -532,7 +555,14 @@ def main():
     ap.add_argument("--no-strong", action="store_true", help="N > 1: skip the strong-scaling sub-result (global batch 32)")
     ap.add_argument("--per-gpu-batch", type=int, default=PER_GPU_BATCH,
                     help="experiments only (host-overhead probes); the reported metric is defined at the default 32")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's losses and a seeded sample of the updated "
+                         "parameters to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of this library's timed path; it does not apply to --impl reference")
     rank = int(os.environ.get("RANK", "0"))
     if args.impl == "reference":
         run_reference(args, rank)

@@ -32,6 +32,33 @@ def perturbed_state_dict(opt, dtype=torch.float64, param_seed=7, bias_seed=11):
     return sd
 
 
+def surface_steps(make_model, make_trainer):
+    """One D half-step with R1 (double backward) and one G half-step of the TINY nets at the perturbed parameters, seeded;
+    returns the losses of both and a checksum of the updated parameters.  ``make_model(opt)`` returns a model wrapper,
+    ``make_trainer(opt, wrapper)`` its training driver.  Run with fp64 as the default dtype."""
+    import contextlib
+    import io
+    from swapping_autoencoder_pytorch_b200 import default_options
+    opt = default_options(**dict(TINY, R1_once_every=1))
+    sd = perturbed_state_dict(opt, dtype=torch.float64)
+    real = rnd(900, 2, 3, 64, 64).clamp(-1, 1)
+    torch.manual_seed(0)
+    with contextlib.redirect_stdout(io.StringIO()):
+        wrapper = make_model(opt)
+    inner = wrapper.singlegpu_model
+    missing, unexpected = inner.load_state_dict(sd, strict=False)
+    assert not unexpected, unexpected
+    trainer = make_trainer(opt, wrapper)
+    torch.manual_seed(1)
+    out = {}
+    for tag in ("D", "G"):
+        losses = trainer.train_one_step({"real_A": real}, 0)
+        out.update({tag + "/" + k: float(v) for k, v in losses.items()})
+    with torch.no_grad():
+        out["param_checksum"] = float(sum(p.double().abs().sum() for p in inner.parameters()))
+    return out
+
+
 def load_golden(name):
     z = np.load(os.path.join(GOLDEN_DIR, name + ".npz"), allow_pickle=False)
     meta = json.loads(str(z["meta"]))

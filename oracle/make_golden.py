@@ -1,16 +1,19 @@
 """ORACLE SUPPORT — generates tests/golden/*.npz by running the REFERENCE ITSELF (native-PyTorch CPU path, fp64).
 
-Run in the build container only (needs the read-only checkout at /root/reference):
-    python oracle/make_golden.py
+Needs a checkout of the reference (``SAE_REFERENCE_ROOT``, see oracle/ref_import.py):
+    python oracle/make_golden.py [ops layers networks surface contract ref_checkpoint ref_surface_steps]
 The fixtures are small (inputs are seeded, parameters are re-derived from a seed by
-``sae_oracle.init_state_dict``; only outputs / gradients are stored) and are committed, so the GPU box — where the
-reference checkout does not exist — can still check the oracle and the CUDA path against the reference's numbers.
+``sae_oracle.init_state_dict``; only outputs / gradients are stored) and are committed, so a machine without the
+reference checkout can still check the oracle and the CUDA path against the reference's numbers.
 """
 import contextlib
+import hashlib
 import io
 import json
 import os
+import subprocess
 import sys
+import tempfile
 
 import numpy as np
 import torch
@@ -272,10 +275,57 @@ def gen_state_dict_contract(R):
         json.dump(contract, f, indent=0, sort_keys=True)
 
 
+def tensor_sha256(t):
+    return hashlib.sha256(t.detach().cpu().contiguous().numpy().tobytes()).hexdigest()
+
+
+def gen_reference_checkpoint(R):
+    """What the reference's own ``BaseModel.save`` (models/base_model.py:33-41) writes for the TINY model at the perturbed
+    fp32 parameters: the directory layout (checkpoint file and ``latest`` symlink), the ordered keys with dtype, shape and
+    SHA-256 of every tensor, the state_dict's ``_metadata``, the full values of the tensors that are not re-derived from the parameter seeds, and the
+    reference encoder's outputs for the seeded image.  The file itself (80 MB) is not stored: the test rebuilds it."""
+    opt = default_options(**TINY)
+    sd = perturbed_state_dict(opt, dtype=torch.float32, param_seed=7, bias_seed=11)
+    with tempfile.TemporaryDirectory() as tmp:
+        opt.checkpoints_dir, opt.name = tmp, "written_by_reference"
+        model = R.sae_model.SwappingAutoencoderModel(opt)
+        with contextlib.redirect_stdout(io.StringIO()):
+            model.initialize()
+        missing, unexpected = model.load_state_dict(sd, strict=False)
+        assert not unexpected, unexpected
+        d = os.path.join(tmp, opt.name)
+        os.makedirs(d)
+        model.save(7000)
+        files = [[f, os.readlink(os.path.join(d, f)) if os.path.islink(os.path.join(d, f)) else None]
+                 for f in sorted(os.listdir(d))]
+        ckpt = torch.load(os.path.join(d, "7k_checkpoint.pth"), map_location="cpu")
+    real = rnd(900, 2, 3, 64, 64).clamp(-1, 1).float()
+    with torch.no_grad():
+        sp, gl = model.E(real)
+    tensors = [[k, str(v.dtype).replace("torch.", ""), list(v.shape), tensor_sha256(v)] for k, v in ckpt.items()]
+    stored = {"stored." + k: v for k, v in ckpt.items() if k not in sd}
+    metadata = [[k, v] for k, v in getattr(ckpt, "_metadata", {}).items()]      # the state_dict's per-module versions
+    save("reference_checkpoint", dict(opt=TINY, param_seed=7, bias_seed=11, real_seed=900, total_steps=7000, files=files,
+                                      tensors=tensors, metadata=metadata), enc_sp=sp, enc_gl=gl, **stored)
+
+
+def gen_reference_surface_steps():
+    """Losses and updated-parameter checksum of the reference's own model / optimizer / network files run over this
+    operator surface (oracle/ref_surface_driver.py, a process of its own)."""
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    res = subprocess.run([sys.executable, os.path.join(root, "oracle", "ref_surface_driver.py"), root,
+                          ref_import.REFERENCE_ROOT], capture_output=True, text=True, check=True, cwd=root)
+    out = json.loads(res.stdout.strip().splitlines()[-1])
+    os.makedirs(OUT, exist_ok=True)
+    with open(os.path.join(OUT, "reference_surface_steps.json"), "w") as f:
+        json.dump({"reference_files": out["reference_files"]}, f, indent=1, sort_keys=True)
+    print("wrote reference_surface_steps", out["reference_files"])
+
+
 def main():
     torch.set_default_dtype(torch.float32)
     R = ref_import.import_reference()
-    which = sys.argv[1:] or ["ops", "layers", "networks", "surface", "contract"]
+    which = sys.argv[1:] or ["ops", "layers", "networks", "surface", "contract", "ref_checkpoint", "ref_surface_steps"]
     if "ops" in which:
         gen_ops(R)
     if "layers" in which:
@@ -286,6 +336,10 @@ def main():
         gen_surface_branches(R)
     if "contract" in which:
         gen_state_dict_contract(R)
+    if "ref_checkpoint" in which:
+        gen_reference_checkpoint(R)
+    if "ref_surface_steps" in which:
+        gen_reference_surface_steps()
 
 
 if __name__ == "__main__":

@@ -20,6 +20,96 @@ int sm_count() {
     return n;
 }
 
+float* det_workspace(size_t nfloats) {
+    constexpr int kMaxDevices = 64;
+    static std::mutex mu;
+    static float* buf[kMaxDevices] = {};
+    static size_t cap[kMaxDevices] = {};
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= kMaxDevices) {
+        fail(SAE_E_CUDA, "deterministic-reduction workspace: no current device");
+        return nullptr;
+    }
+    std::lock_guard<std::mutex> lock(mu);
+    if (cap[dev] < nfloats) {
+        // Allocated on first use, at least 64 MB: enough for every reduction of the default 256x256 training step.  The eager
+        // half-steps that precede a graph capture size it; a capture that needed more would fail at cudaMalloc, and graphs.py
+        // then runs that half-step eagerly.
+        size_t want = nfloats + nfloats / 4;
+        if (want < ((size_t)16 << 20)) want = (size_t)16 << 20;
+        void* p = nullptr;
+        cudaError_t e = cudaMalloc(&p, want * sizeof(float));
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            fail(SAE_E_CUDA, "deterministic-reduction workspace of %zu bytes: %s", want * sizeof(float), cudaGetErrorString(e));
+            return nullptr;
+        }
+        buf[dev] = static_cast<float*>(p);     // the previous buffer stays allocated: captured graphs may still use it
+        cap[dev] = want;
+    }
+    return buf[dev];
+}
+
+constexpr int DR_COLS = 32, DR_MAX_ROWS = 8;
+
+// grid = (column blocks, part groups), block = (32, rows).  Group g sums parts [g * per, min(parts, (g + 1) * per)): row r takes
+// every rows-th part from g * per + r, then row 0 adds the rows in order.  With ws2 the group sums go to ws2[g * n + c],
+// otherwise (one group) they are added to the destination.
+__global__ void det_reduce_kernel(const float* __restrict__ ws, int64_t n, int parts, int per, float* __restrict__ ws2,
+                                  float* a, int64_t n_a, float* b) {
+    __shared__ float red[DR_MAX_ROWS][DR_COLS + 1];
+    const int64_t col = (int64_t)blockIdx.x * DR_COLS + threadIdx.x;
+    const int b0 = (int)blockIdx.y * per;
+    const int b1 = min(b0 + per, parts);
+    float s = 0.f;
+    if (col < n)
+        for (int k = b0 + (int)threadIdx.y; k < b1; k += (int)blockDim.y) s += ws[(int64_t)k * n + col];
+    red[threadIdx.y][threadIdx.x] = s;
+    __syncthreads();
+    if (threadIdx.y != 0 || col >= n) return;
+    float t = red[0][threadIdx.x];
+    for (int r = 1; r < (int)blockDim.y; ++r) t += red[r][threadIdx.x];
+    if (ws2 != nullptr) {
+        ws2[(int64_t)blockIdx.y * n + col] = t;
+        return;
+    }
+    float* dst = col < n_a ? (a ? a + col : nullptr) : (b ? b + (col - n_a) : nullptr);
+    if (dst) *dst += t;
+}
+
+static int det_groups(int64_t n, int parts) {
+    // many parts over few columns (per-block bias sums): a first pass over part groups fills the machine
+    if (parts <= 64) return 1;
+    const int64_t col_blocks = (n + DR_COLS - 1) / DR_COLS;
+    int64_t g = ((int64_t)sm_count() * 4 + col_blocks - 1) / col_blocks;
+    if (g > parts / 32) g = parts / 32;
+    return g < 1 ? 1 : (int)g;
+}
+
+size_t det_reduce_floats(int64_t n, int parts) {
+    const int g = det_groups(n, parts);
+    return (size_t)parts * n + (g > 1 ? (size_t)g * n : 0);
+}
+
+int det_reduce(float* a, int64_t n_a, float* b, const float* ws, int64_t n, int parts, cudaStream_t st) {
+    if (n <= 0 || parts <= 0) return SAE_OK;
+    int g = det_groups(n, parts);
+    const int per = (parts + g - 1) / g;
+    g = (parts + per - 1) / per;
+    const unsigned col_blocks = (unsigned)((n + DR_COLS - 1) / DR_COLS);
+    if (g > 1) {
+        float* ws2 = const_cast<float*>(ws) + (int64_t)parts * n;
+        det_reduce_kernel<<<dim3(col_blocks, (unsigned)g), dim3(DR_COLS, DR_MAX_ROWS), 0, st>>>(ws, n, parts, per, ws2, a, n_a, b);
+        int rc = check_launch("det_reduce (groups)");
+        if (rc) return rc;
+        ws = ws2;
+        parts = g;
+    }
+    const unsigned rows = (unsigned)(parts < DR_MAX_ROWS ? parts : DR_MAX_ROWS);
+    det_reduce_kernel<<<dim3(col_blocks, 1), dim3(DR_COLS, rows), 0, st>>>(ws, n, parts, parts, nullptr, a, n_a, b);
+    return check_launch("det_reduce");
+}
+
 static int validate_geom(const sae_conv_geom* g, const char* who) {
     if (!g) return fail(SAE_E_INVALID, "%s: null geometry", who);
     if (g->N < 0 || g->H <= 0 || g->W <= 0 || g->C <= 0 || g->K <= 0 || g->R <= 0 || g->S <= 0 || g->P <= 0 ||

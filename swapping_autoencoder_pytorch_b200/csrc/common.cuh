@@ -39,6 +39,24 @@ inline int check_launch(const char* what) {
 // process drives one GPU in this design).
 int sm_count();
 
+// Deterministic cross-block reductions.  Float atomics add in whatever order the blocks happen to finish, so the last bits
+// of a reduced gradient — and, through the optimiser, every later training step — would change from run to run.  Instead,
+// every block writes its partial sums to its own slice of a workspace with plain stores, and det_reduce adds the slices
+// in index order.
+//
+// det_workspace: a device buffer of at least nfloats floats, library-owned and grow-only.  A buffer is never freed once
+// handed out, because captured CUDA graphs keep its address; all users run in stream order, one after the other.
+// Returns nullptr (and sets the error text) when the allocation fails.
+float* det_workspace(size_t nfloats);
+// out[c] += sum over b = 0 .. parts-1 (in that order) of ws[b * n + c], for c < n; columns c < n_a go to a[c] (skipped if
+// a is null), the rest to b[c - n_a] (skipped if b is null).  ws must come from det_workspace(det_reduce_floats(n, parts)):
+// the reduction uses the space behind the parts * n partials.
+size_t det_reduce_floats(int64_t n, int parts);
+int det_reduce(float* a, int64_t n_a, float* b, const float* ws, int64_t n, int parts, cudaStream_t st);
+inline int det_reduce(float* out, const float* ws, int64_t n, int parts, cudaStream_t st) {
+    return det_reduce(out, n, nullptr, ws, n, parts, st);
+}
+
 __device__ __forceinline__ float rna_tf32(float v) {
     uint32_t r;
     asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(v));

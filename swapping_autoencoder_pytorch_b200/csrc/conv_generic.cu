@@ -9,7 +9,7 @@
 //   iy = (oy*SY + OFFY + r*DY) / DIV  (only if divisible and in range), same in x.
 //   fprop: SY = stride, DY = +1, OFF = -pad, DIV = 1;  dgrad: SY = 1, DY = -1, OFF = +pad, DIV = stride.
 // wgrad:  dW[o, (r,s,c)] += sum_pixels dy[pixel, o] * x_gathered[pixel, (r,s,c)], split over pixels,
-//   fp32 atomics into dW.
+//   each split writes its partial dW to its own workspace slice; det_reduce adds the slices in split order.
 // Operands are rounded to TF32 (cvt.rna) when fragments are loaded, accumulation is fp32.
 #include "conv_internal.cuh"
 
@@ -60,7 +60,7 @@ conv_gather_kernel(const float* __restrict__ src, const float* __restrict__ wmat
     const int n0 = blockIdx.y * BN;
     const int KB_total = (p.K + BK - 1) / BK;
     // split-K (gridDim.z > 1, small-M GEMMs such as the style / head linears): this CTA reduces k-blocks
-    // [kb_begin, kb_begin + KB) and adds its partial tile to the zero-initialised output with fp32 atomics
+    // [kb_begin, kb_begin + KB) and writes its partial tile to slice blockIdx.z of the workspace ``out`` points to
     const int kb_per = (KB_total + (int)gridDim.z - 1) / (int)gridDim.z;
     const int kb_begin = (int)blockIdx.z * kb_per;
     const int KB = max(0, min(kb_per, KB_total - kb_begin));
@@ -214,7 +214,7 @@ conv_gather_kernel(const float* __restrict__ src, const float* __restrict__ wmat
 #pragma unroll
                     for (int u = 0; u < 2; ++u) {
                         int col = n0 + wn * 32 + j * 8 + 2 * t + u;
-                        if (col < p.Ncol) atomicAdd(out + m * p.Ncol + col, acc[i][j][h * 2 + u]);
+                        if (col < p.Ncol) out[((int64_t)blockIdx.z * p.M + m) * p.Ncol + col] = acc[i][j][h * 2 + u];
                     }
             }
         return;
@@ -444,7 +444,7 @@ conv_wgrad_kernel(const float* __restrict__ dy, const float* __restrict__ x, flo
 #pragma unroll
                 for (int u = 0; u < 2; ++u) {
                     int n = n0 + wn * 32 + j * 8 + 2 * t + u;
-                    if (n < p.Ncol) atomicAdd(dw + (int64_t)o * p.Ncol + n, acc[i][j][h * 2 + u]);
+                    if (n < p.Ncol) dw[((int64_t)blockIdx.z * p.Ko + o) * p.Ncol + n] = acc[i][j][h * 2 + u];
                 }
         }
 }
@@ -466,13 +466,20 @@ static int launch_gather(const float* src, const float* wmat, float* out, const 
     if (plain && grid.x * grid.y <= 16 && kblocks >= 16) {
         unsigned z = (unsigned)(kblocks / 4);
         if (z > 32) z = 32;
-        if (z > 1) {
-            grid.z = z;
-            SAE_CUDA_TRY(cudaMemsetAsync(out, 0, (size_t)p.M * p.Ncol * sizeof(float), st));
-        }
+        if (z > 1) grid.z = z;
     }
-    conv_gather_kernel<BN, VEC><<<grid, NTHREADS, smem, st>>>(src, wmat, out, p, e);
-    return check_launch("conv_gather");
+    if (grid.z == 1) {
+        conv_gather_kernel<BN, VEC><<<grid, NTHREADS, smem, st>>>(src, wmat, out, p, e);
+        return check_launch("conv_gather");
+    }
+    // split K: per-split partial tiles, then the output = their sum in split order
+    float* part = det_workspace(det_reduce_floats(p.M * p.Ncol, (int)grid.z));
+    if (!part) return SAE_E_CUDA;
+    SAE_CUDA_TRY(cudaMemsetAsync(out, 0, (size_t)p.M * p.Ncol * sizeof(float), st));
+    conv_gather_kernel<BN, VEC><<<grid, NTHREADS, smem, st>>>(src, wmat, part, p, e);
+    int rc = check_launch("conv_gather");
+    if (rc) return rc;
+    return det_reduce(out, part, p.M * p.Ncol, (int)grid.z, st);
 }
 
 int conv_gather_dispatch(const float* src, const float* wmat, float* out, const GatherParams& p, const EpiParams& e,
@@ -494,8 +501,12 @@ static int launch_wgrad(const float* dy, const float* x, float* dw, const WgradP
         attr_done = true;
     }
     dim3 grid((unsigned)((p.Ko + 127) / 128), (unsigned)((p.Ncol + 127) / 128), splits);
-    conv_wgrad_kernel<VA, VB><<<grid, NTHREADS, smem, st>>>(dy, x, dw, p);
-    return check_launch("conv_wgrad");
+    float* part = det_workspace(det_reduce_floats((int64_t)p.Ko * p.Ncol, (int)splits));
+    if (!part) return SAE_E_CUDA;
+    conv_wgrad_kernel<VA, VB><<<grid, NTHREADS, smem, st>>>(dy, x, part, p);
+    int rc = check_launch("conv_wgrad");
+    if (rc) return rc;
+    return det_reduce(dw, part, (int64_t)p.Ko * p.Ncol, (int)splits, st);
 }
 
 int conv_wgrad_generic(const float* dy, const float* x, float* dw, const sae_conv_geom* g, cudaStream_t st) {

@@ -71,19 +71,18 @@ bias_act_kernel(const float* __restrict__ x, const float* __restrict__ b, const 
 // ---------------------------------------------------------------------------- bias_act backward
 // grad_in = grad_out * mask(out) * scale; grad_bias[c] += sum(grad_in); channels innermost.
 // Every thread keeps a fixed channel group across its grid-stride loop (stride is a multiple of
-// the number of channel groups), accumulates in registers, then one shared-memory reduction and
-// one global atomic per channel per CTA.
+// the number of channel groups) and accumulates in registers.  The CTA then sums each channel over its
+// threads in thread order and writes the sums (and the noise-weight sum) to its own row part[blockIdx.x][C + 1];
+// det_reduce adds the rows in order.
 template <int VEC>
 __global__ void __launch_bounds__(256)
 bias_act_bwd_kernel(const float* __restrict__ go, const float* __restrict__ outp, float* __restrict__ gi,
-                    float* __restrict__ gb, int64_t size_v, int cv, int64_t stride_v,
+                    float* __restrict__ part, int want_gb, int64_t size_v, int cv, int64_t stride_v,
                     float alpha, float scale,
-                    const float* __restrict__ noise, int64_t noise_div, float* __restrict__ gnw, int round_tf32,
+                    const float* __restrict__ noise, int64_t noise_div, int round_tf32,
                     const uint32_t* __restrict__ act_mask) {
-    extern __shared__ float sacc[];   // [cv * VEC] (+1 slot for the noise-weight grad)
+    extern __shared__ float sthr[];   // [blockDim.x * VEC] per-thread channel sums, then [blockDim.x / 32] warp noise sums
     const int C = cv * VEC;
-    for (int i = threadIdx.x; i <= C; i += blockDim.x) sacc[i] = 0.f;
-    __syncthreads();
 
     const int64_t tid = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     float bsum[VEC];
@@ -119,23 +118,29 @@ bias_act_bwd_kernel(const float* __restrict__ go, const float* __restrict__ outp
             if (VEC == 4) reinterpret_cast<float4*>(gi)[i] = make_float4(g[0], g[1 % VEC], g[2 % VEC], g[3 % VEC]);
             else gi[i] = g[0];
         }
-        if (gb) {
-            const int c0 = (int)(tid % cv) * VEC;
+    }
 #pragma unroll
-            for (int j = 0; j < VEC; ++j) atomicAdd(&sacc[c0 + j], bsum[j]);
-        }
-    }
-    if (noise) {
-        nsum = warp_sum(nsum);
-        if ((threadIdx.x & 31) == 0) atomicAdd(&sacc[C], nsum);
-    }
+    for (int j = 0; j < VEC; ++j) sthr[threadIdx.x * VEC + j] = bsum[j];
+    float* swarp = sthr + blockDim.x * VEC;
+    nsum = warp_sum(nsum);
+    if ((threadIdx.x & 31) == 0) swarp[threadIdx.x >> 5] = nsum;
     __syncthreads();
-    if (gb)
+    float* row = part + (int64_t)blockIdx.x * (C + 1);
+    if (want_gb) {
+        // thread t of this CTA holds channel group (blockIdx.x * blockDim.x + t) % cv
+        const int shift = (int)(((int64_t)blockIdx.x * blockDim.x) % cv);
         for (int i = threadIdx.x; i < C; i += blockDim.x) {
-            float v = sacc[i];
-            if (v != 0.f) atomicAdd(gb + i, v);
+            const int cg = i / VEC, j = i - cg * VEC;
+            float v = 0.f;
+            for (int t = (cg - shift + cv) % cv; t < (int)blockDim.x; t += cv) v += sthr[t * VEC + j];
+            row[i] = v;
         }
-    if (noise && threadIdx.x == 0) atomicAdd(gnw, sacc[C]);
+    }
+    if (noise && threadIdx.x == 0) {
+        float v = 0.f;
+        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) v += swarp[w];
+        row[C] = v;
+    }
 }
 
 // ------------------------------------------------------------------------------------ modulate
@@ -168,15 +173,14 @@ modulate_scalar_kernel(const float* __restrict__ x, const float* __restrict__ s,
 }
 
 // dx = dy * s;  ds[n, c] += sum_hw dy * x.   grid = (chunks, N); each CTA covers a pixel range of one
-// sample; thread keeps a fixed channel group; smem reduce then one atomic per channel per CTA.
+// sample; thread keeps a fixed channel group, the CTA sums each channel over its threads in thread order and
+// writes the sums to its own row part[blockIdx.x][n][C]; det_reduce adds the rows in order.
 template <int VEC>
 __global__ void __launch_bounds__(256)
 modulate_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ x, const float* __restrict__ s,
-                    float* __restrict__ dx, float* __restrict__ ds, int64_t hw, int cv, int64_t pix_per_cta, int round_tf32) {
-    extern __shared__ float sacc[];   // [cv*VEC]
+                    float* __restrict__ dx, float* __restrict__ part, int64_t hw, int cv, int64_t pix_per_cta, int round_tf32) {
+    extern __shared__ float sthr[];   // [blockDim.x * VEC]
     const int C = cv * VEC;
-    for (int i = threadIdx.x; i < C; i += blockDim.x) sacc[i] = 0.f;
-    __syncthreads();
     const int n = blockIdx.y;
     const int64_t p0 = blockIdx.x * pix_per_cta;
     int64_t p1 = p0 + pix_per_cta;
@@ -184,10 +188,11 @@ modulate_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ x, c
     const int64_t base_v = (int64_t)n * hw * cv;
     const int64_t lo = p0 * cv, hi = p1 * cv;          // in VEC units inside this sample
     const int64_t stride = (blockDim.x / cv > 0) ? (int64_t)(blockDim.x / cv) * cv : 0;
-    float acc[VEC];
-#pragma unroll
-    for (int j = 0; j < VEC; ++j) acc[j] = 0.f;
+    float* row = part + ((int64_t)blockIdx.x * gridDim.y + n) * C;
     if (stride > 0) {
+        float acc[VEC];
+#pragma unroll
+        for (int j = 0; j < VEC; ++j) acc[j] = 0.f;
         if (threadIdx.x < stride) {
             const int c = threadIdx.x % cv;
             float m[VEC];
@@ -211,27 +216,37 @@ modulate_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ x, c
                 if (VEC == 4) reinterpret_cast<float4*>(dx)[base_v + i] = make_float4(g[0], g[1 % VEC], g[2 % VEC], g[3 % VEC]);
                 else dx[base_v + i] = g[0];
             }
+        }
 #pragma unroll
-            for (int j = 0; j < VEC; ++j) atomicAdd(&sacc[c * VEC + j], acc[j]);
+        for (int j = 0; j < VEC; ++j) sthr[threadIdx.x * VEC + j] = acc[j];
+        __syncthreads();
+        // thread t < stride holds channel group t % cv
+        for (int i = threadIdx.x; i < C; i += blockDim.x) {
+            const int cg = i / VEC, j = i - cg * VEC;
+            float v = 0.f;
+            for (int t = cg; t < stride; t += cv) v += sthr[t * VEC + j];
+            row[i] = v;
         }
     } else {
-        // more channel groups than threads: each thread walks several channel groups per pixel
-        for (int64_t i = lo + threadIdx.x; i < hi; i += blockDim.x) {
-            const int c = (int)(i % cv);
+        // more channel groups than threads: each thread owns whole channel groups and walks the pixels of the range
+        for (int cc = threadIdx.x; cc < cv; cc += blockDim.x) {
+            float acc[VEC];
 #pragma unroll
-            for (int j = 0; j < VEC; ++j) {
-                int64_t e = (base_v + i) * VEC + j;
-                float g = dy[e], a = x[e];
-                atomicAdd(&sacc[c * VEC + j], g * a);
-                float d = g * __ldg(s + (int64_t)n * C + c * VEC + j);
-                dx[e] = round_tf32 ? rna_tf32(d) : d;
+            for (int j = 0; j < VEC; ++j) acc[j] = 0.f;
+            for (int64_t pp = p0; pp < p1; ++pp) {
+                const int64_t i = pp * cv + cc;
+#pragma unroll
+                for (int j = 0; j < VEC; ++j) {
+                    int64_t e = (base_v + i) * VEC + j;
+                    float g = dy[e], a = x[e];
+                    acc[j] = fmaf(g, a, acc[j]);
+                    float d = g * __ldg(s + (int64_t)n * C + cc * VEC + j);
+                    dx[e] = round_tf32 ? rna_tf32(d) : d;
+                }
             }
+#pragma unroll
+            for (int j = 0; j < VEC; ++j) row[cc * VEC + j] = acc[j];
         }
-    }
-    __syncthreads();
-    for (int i = threadIdx.x; i < C; i += blockDim.x) {
-        float v = sacc[i];
-        if (v != 0.f) atomicAdd(ds + (int64_t)n * C + i, v);
     }
 }
 
@@ -544,17 +559,21 @@ extern "C" int sae_bias_act_backward(const float* grad_out, const float* out, fl
         threads = (int64_t)blocks * 256;
         stride = (threads / cv) * cv;
     }
-    size_t smem = (size_t)(size_b + 1) * sizeof(float);
-    if (vec) {
-        if (smem > 48 * 1024) cudaFuncSetAttribute(bias_act_bwd_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        bias_act_bwd_kernel<4><<<blocks, 256, smem, st>>>(grad_out, out, grad_in, grad_bias, size_v, cv, stride, alpha, scale,
-                                                         noise, noise_div, grad_noise_weight, round_tf32, act_mask);
-    } else {
-        if (smem > 48 * 1024) cudaFuncSetAttribute(bias_act_bwd_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        bias_act_bwd_kernel<1><<<blocks, 256, smem, st>>>(grad_out, out, grad_in, grad_bias, size_v, cv, stride, alpha, scale,
-                                                         noise, noise_div, grad_noise_weight, round_tf32, nullptr);
+    float* part = nullptr;
+    if (grad_bias || noise) {
+        part = det_workspace(det_reduce_floats(size_b + 1, (int)blocks));
+        if (!part) return SAE_E_CUDA;
     }
-    return check_launch("bias_act_backward");
+    const size_t smem = (size_t)(256 * V + 256 / 32) * sizeof(float);
+    if (vec)
+        bias_act_bwd_kernel<4><<<blocks, 256, smem, st>>>(grad_out, out, grad_in, part, grad_bias != nullptr, size_v, cv, stride, alpha,
+                                                         scale, noise, noise_div, round_tf32, act_mask);
+    else
+        bias_act_bwd_kernel<1><<<blocks, 256, smem, st>>>(grad_out, out, grad_in, part, grad_bias != nullptr, size_v, cv, stride, alpha,
+                                                         scale, noise, noise_div, round_tf32, nullptr);
+    int rc = check_launch("bias_act_backward");
+    if (rc || !part) return rc;
+    return det_reduce(grad_bias, size_b, noise ? grad_noise_weight : nullptr, part, size_b + 1, (int)blocks, st);
 }
 
 extern "C" int sae_modulate(const float* x, const float* s, float* out, int n, int64_t hw, int c, int round_tf32,
@@ -594,10 +613,14 @@ extern "C" int sae_modulate_backward(const float* dy, const float* x, const floa
     if (pix_per_cta < 8) pix_per_cta = 8;
     unsigned chunks = (unsigned)((hw + pix_per_cta - 1) / pix_per_cta);
     dim3 grid(chunks, (unsigned)n);
-    size_t smem = (size_t)c * sizeof(float);
-    if (vec) modulate_bwd_kernel<4><<<grid, 256, smem, st>>>(dy, x, s, dx, ds, hw, c / V, pix_per_cta, round_tf32);
-    else     modulate_bwd_kernel<1><<<grid, 256, smem, st>>>(dy, x, s, dx, ds, hw, c / V, pix_per_cta, round_tf32);
-    return check_launch("modulate_backward");
+    float* part = det_workspace(det_reduce_floats((int64_t)n * c, (int)chunks));
+    if (!part) return SAE_E_CUDA;
+    const size_t smem = (size_t)256 * V * sizeof(float);
+    if (vec) modulate_bwd_kernel<4><<<grid, 256, smem, st>>>(dy, x, s, dx, part, hw, c / V, pix_per_cta, round_tf32);
+    else     modulate_bwd_kernel<1><<<grid, 256, smem, st>>>(dy, x, s, dx, part, hw, c / V, pix_per_cta, round_tf32);
+    int rc = check_launch("modulate_backward");
+    if (rc) return rc;
+    return det_reduce(ds, part, (int64_t)n * c, (int)chunks, st);
 }
 
 extern "C" int sae_add_scale(const float* a, const float* b, float* out, int64_t n, float scale, int round_tf32, void* stream) {

@@ -9,7 +9,7 @@
 // N = 4.  Here x is read ONCE: a warp owns a strip of pixels of one sample, lane l holds the 3 x 4 combined weights
 // s[n, c] * w[o, c] of its four channels c = 4l + 128j in registers, reads its float4 of every pixel and the three partial
 // sums are reduced with shuffles.  Backward, also one pass over x: dx = sum_o dy[o] * s * w (written) and the per-sample
-// weight gradient G[n, o, c] = sum_p dy[n, p, o] x[n, p, c] (registers -> one atomic flush per warp), from which the caller
+// weight gradient G[n, o, c] = sum_p dy[n, p, o] x[n, p, c] (registers -> one row of partial sums per strip, added in strip order), from which the caller
 // forms ds = sum_o G * w and dw = sum_n G * s on [N, 3, C] values.
 #include "common.cuh"
 
@@ -147,7 +147,7 @@ torgb_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ x, cons
                 for (int o = 0; o < 3; ++o)
 #pragma unroll
                     for (int u = 0; u < 4; ++u)
-                        if (c + u < C) atomicAdd(gw + ((int64_t)n * 3 + o) * C + c + u, g[j][o][u]);
+                        if (c + u < C) gw[(((item % strips_per_sample) * N + n) * 3 + o) * C + c + u] = g[j][o][u];
             }
         }
     }
@@ -206,7 +206,13 @@ extern "C" int sae_torgb_backward(const float* dy, const float* x, const float* 
     if (blocks > cap) blocks = cap;
     const int nj = (C + 127) / 128;
     cudaStream_t st = (cudaStream_t)stream;
-#define SAE_TORGB_BWD(NJ) torgb_bwd_kernel<NJ><<<(unsigned)blocks, 256, 0, st>>>(dy, x, s, w, dx, gw, N, HW, W, C, strips, wscale, ds_n, ds_c, ds_h, ds_w, round_tf32)
+    // gw: one row of partial sums per strip, [strip][N][3][C], added in strip order after the kernel
+    float* part = nullptr;
+    if (gw) {
+        part = det_workspace(det_reduce_floats((int64_t)N * 3 * C, strips));
+        if (!part) return SAE_E_CUDA;
+    }
+#define SAE_TORGB_BWD(NJ) torgb_bwd_kernel<NJ><<<(unsigned)blocks, 256, 0, st>>>(dy, x, s, w, dx, part, N, HW, W, C, strips, wscale, ds_n, ds_c, ds_h, ds_w, round_tf32)
     switch (nj) {
         case 1: SAE_TORGB_BWD(1); break;
         case 2: SAE_TORGB_BWD(2); break;
@@ -214,5 +220,7 @@ extern "C" int sae_torgb_backward(const float* dy, const float* x, const float* 
         default: SAE_TORGB_BWD(8); break;
     }
 #undef SAE_TORGB_BWD
-    return check_launch("torgb_backward");
+    int rc = check_launch("torgb_backward");
+    if (rc || !gw) return rc;
+    return det_reduce(gw, part, (int64_t)N * 3 * C, strips, st);
 }

@@ -246,10 +246,11 @@ constexpr int FT_W = 16, FT_H = 16;
 
 // MASK variant (sae_fir_act_backward): the FIR result is the gradient arriving at a fused bias + leaky-ReLU, so the store
 // applies that activation's backward — times (act_out > 0 ? 1 : alpha) * scale — and the per-channel sums of the masked
-// gradient (the bias gradient) are reduced CTA-wide in shared memory and added to grad_bias with 32 atomics per CTA.
+// gradient (the bias gradient) are reduced CTA-wide in shared memory, in a fixed order, and written to the CTA's row of
+// partial sums; the caller adds the rows in order (det_reduce).
 struct FirMask {
     const float* act_out;     // saved activation output, same shape as the FIR output
-    float* grad_bias;         // [minor], accumulated; may be null
+    float* grad_bias;         // partial sums [(n * tiles_y + ty) * tiles_x + tx][minor], one row per pixel tile; may be null
     float alpha, scale;
     // MODE 2 (sae_fir_bias_act, forward): out = lrelu(FIR(x) + noise_weight * noise[pixel] + bias[c]) * scale
     const float* bias;        // [minor] or null
@@ -268,8 +269,7 @@ fir_tma_kernel(const __grid_constant__ CUtensorMap map_x, float* __restrict__ ou
     extern __shared__ uint8_t fir_smem[];
     __shared__ __align__(8) uint64_t bar_storage;
     constexpr bool MASK = MODE == 1;
-    __shared__ float bias_part[32];
-    if (MASK && threadIdx.x < 32) bias_part[threadIdx.x] = 0.f;
+    __shared__ float bias_part[8][32];     // per warp
     const uint32_t base = (smem_u32(fir_smem) + 127u) & ~127u;
     const float4* win = reinterpret_cast<const float4*>(fir_smem + (base - smem_u32(fir_smem)));
     const uint32_t bar = smem_u32(&bar_storage);
@@ -365,18 +365,23 @@ fir_tma_kernel(const __grid_constant__ CUtensorMap map_x, float* __restrict__ ou
     }
     if (MASK && mk.grad_bias != nullptr) {
         // the 32 threads that share cvec sit in the lanes {cvec, cvec + 8, cvec + 16, cvec + 24} of every warp: fold those
-        // four with shuffles, then one shared-memory atomic per warp and channel, then 32 global atomics per CTA
+        // four with shuffles, then one shared-memory slot per warp and channel, summed over the warps in order
 #pragma unroll
         for (int o = 8; o < 32; o <<= 1) {
             bsum.x += __shfl_xor_sync(0xffffffffu, bsum.x, o); bsum.y += __shfl_xor_sync(0xffffffffu, bsum.y, o);
             bsum.z += __shfl_xor_sync(0xffffffffu, bsum.z, o); bsum.w += __shfl_xor_sync(0xffffffffu, bsum.w, o);
         }
         if ((threadIdx.x & 31) < 8) {
-            atomicAdd(&bias_part[cvec * 4 + 0], bsum.x); atomicAdd(&bias_part[cvec * 4 + 1], bsum.y);
-            atomicAdd(&bias_part[cvec * 4 + 2], bsum.z); atomicAdd(&bias_part[cvec * 4 + 3], bsum.w);
+            float* wp = bias_part[threadIdx.x >> 5];
+            wp[cvec * 4 + 0] = bsum.x; wp[cvec * 4 + 1] = bsum.y; wp[cvec * 4 + 2] = bsum.z; wp[cvec * 4 + 3] = bsum.w;
         }
         __syncthreads();
-        if (threadIdx.x < 32) atomicAdd(mk.grad_bias + cb * 32 + threadIdx.x, bias_part[threadIdx.x]);
+        if (threadIdx.x < 32) {
+            float v = 0.f;
+#pragma unroll
+            for (int w = 0; w < 8; ++w) v += bias_part[w][threadIdx.x];
+            mk.grad_bias[(((int64_t)n * tiles_y + ty) * tiles_x + tx) * p.minor + cb * 32 + threadIdx.x] = v;
+        }
     }
 }
 
@@ -597,9 +602,16 @@ extern "C" int sae_fir_act_backward(const float* grad, const float* taps_y, cons
     mk.act_out = act_out; mk.grad_bias = grad_bias; mk.alpha = alpha; mk.scale = scale; mk.act_mask = const_cast<uint32_t*>(act_mask);
     cudaStream_t st = (cudaStream_t)stream;
     mk.bias = nullptr; mk.noise = nullptr; mk.noise_weight = nullptr;
+    const int parts = (int)(major * ((p.out_w + FT_W - 1) / FT_W) * ((p.out_h + FT_H - 1) / FT_H));
+    if (grad_bias) {
+        mk.grad_bias = det_workspace(det_reduce_floats(minor, parts));
+        if (!mk.grad_bias) return SAE_E_CUDA;
+    }
     int rc = kernel_h == 3 ? launch_tma<3, 3, 1>(grad, grad_in, p, t, st, mk) : launch_tma<4, 4, 1>(grad, grad_in, p, t, st, mk);
     if (rc) return rc;
-    return check_launch("fir_act_backward");
+    rc = check_launch("fir_act_backward");
+    if (rc || !grad_bias) return rc;
+    return det_reduce(grad_bias, mk.grad_bias, minor, parts, st);
 }
 
 // FIR (up = down = 1, separable 3 or 4 taps) followed by NoiseInjection + bias + leaky-ReLU in ONE pass:

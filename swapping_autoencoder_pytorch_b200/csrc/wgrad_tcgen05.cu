@@ -15,8 +15,9 @@
 //   * layers with 256 out channels per tile pair run as CTA pairs (cta_group::2, wgrad_tc_kernel<2>): half of every x tile
 //     per CTA, a 5-deep ring
 //   * one TMEM accumulator (128 x 128 fp32 = 128 columns) per tap; the dy tile is reused by all taps of the group
-//   * grid = (M tiles x N tiles, tap groups, pixel splits); partial sums are reduced with vectorised fp32 atomics
-//     (red.global.add.v4.f32) straight from the TMEM read — dW must be zero-initialised by the caller.
+//   * grid = (M tiles x N tiles, tap groups, pixel splits); every split stores its partial dW straight from the TMEM read
+//     into its own workspace slice, and det_reduce adds the slices to dW in split order (no float atomics: the result is
+//     the same from run to run).
 #include "tc_common.cuh"
 
 namespace sae {
@@ -49,7 +50,9 @@ struct WgParams {
     int chunks_per_image;            // > 0 selects that mode (tn == 1)
     const float* mod_s;              // [N, C]
     const float* mod_w;              // [Ko, taps, C], the filter the forward pass used
-    float* mod_ds;                   // [N, C], accumulated
+    float* mod_ds;                   // partial terms [img][split - first split of img][out tile][tap group][warp][C]
+    int ds_kmax, ds_tiles_o;         // extents of those partials: splits per image, 128-row output tiles
+    int64_t dw_numel;                // Ko * taps * C: one workspace slice of partial dW
     int five_d;                      // pair mode: the tensor maps are the 5-D views (one TMA instruction per operand tile)
 };
 
@@ -299,16 +302,26 @@ wgrad_tc_kernel(const __grid_constant__ CUtensorMap map_dy, const __grid_constan
                         for (int j = 0; j < 32; ++j) {
                             float t = in_range ? v[j] * __ldg(p.mod_w + off + j) : 0.f;
                             t = warp_sum(t);
-                            if (lane == 0 && c < p.C) atomicAdd(p.mod_ds + (int64_t)img * p.C + c + j, t);
+                            if (lane == 0 && c < p.C) {
+                                // the first tap of this CTA's group stores, the others add (same thread, fixed order)
+                                float* d = p.mod_ds + ((((int64_t)img * p.ds_kmax + (int)blockIdx.z - (int)(((int64_t)img * p.chunks_per_image) / p.chunks_per_split))
+                                                        * p.ds_tiles_o + o0 / 128) * gridDim.y + blockIdx.y) * 4 * p.C + (int64_t)lg * p.C + c + j;
+                                *d = q < p.cpt ? t : *d + t;
+                            }
                             v[j] *= (c < p.C) ? __ldg(sv + j) : 0.f;
                         }
                     }
                     if (in_range) {
-                        float* dst = dw + off;
+                        // this split's slice; later segments (images) of the same CTA add to what the first one stored
+                        float4* dst = reinterpret_cast<float4*>(dw + (int64_t)blockIdx.z * p.dw_numel + off);
 #pragma unroll
                         for (int j = 0; j < 8; ++j) {
-                            asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + 4 * j), "f"(v[4 * j]),
-                                         "f"(v[4 * j + 1]), "f"(v[4 * j + 2]), "f"(v[4 * j + 3]) : "memory");
+                            float4 a = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
+                            if (seg > 0) {
+                                const float4 b = dst[j];
+                                a.x += b.x; a.y += b.y; a.z += b.z; a.w += b.w;
+                            }
+                            dst[j] = a;
                         }
                     }
                 }
@@ -447,10 +460,9 @@ wgrad_narrow_kernel(const __grid_constant__ CUtensorMap map_dy, const __grid_con
                     float v[32];
                     tmem_ld32(tmem_base + ((uint32_t)(lg * 32) << 16) + (uint32_t)(r * p.Ko + nb * 32), v);
                     if (lg < p.S) {
-                        float* dst = dw + (int64_t)(nb * 32) * ld + (int64_t)(r * p.S + lg) * p.C + lane;
+                        float* dst = dw + (int64_t)blockIdx.x * p.dw_numel + (int64_t)(nb * 32) * ld + (int64_t)(r * p.S + lg) * p.C + lane;
 #pragma unroll
-                        for (int i = 0; i < 32; ++i)
-                            asm volatile("red.global.add.f32 [%0], %1;" ::"l"(dst + (int64_t)i * ld), "f"(v[i]) : "memory");
+                        for (int i = 0; i < 32; ++i) dst[(int64_t)i * ld] = v[i];
                     }
                 }
         }
@@ -491,6 +503,25 @@ int tc_wgrad_modulated(const float* dy, const float* x, const float* s, const fl
     return tc_wgrad_impl(dy, x, dw, g, st, s, w_krsc, ds);
 }
 
+// ds[img, c] += the style-gradient terms of every CTA that drained image img, summed in a fixed order: the splits that cover
+// the image, then output tiles, tap groups and warps
+__global__ void mod_ds_reduce_kernel(const float* __restrict__ part, float* __restrict__ ds, int N, int C, int kmax, int tiles_o,
+                                     int groups, int chunks_per_image, int chunks_per_split, int splits) {
+    const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= (int64_t)N * C) return;
+    const int img = (int)(idx / C), c = (int)(idx % C);
+    const int first = (int)(((int64_t)img * chunks_per_image) / chunks_per_split);
+    int last = (int)(((int64_t)(img + 1) * chunks_per_image - 1) / chunks_per_split);
+    if (last > splits - 1) last = splits - 1;
+    float v = 0.f;
+    for (int k = 0; k <= last - first; ++k)
+        for (int o = 0; o < tiles_o; ++o)
+            for (int y = 0; y < groups; ++y)
+                for (int lg = 0; lg < 4; ++lg)
+                    v += part[(((((int64_t)img * kmax + k) * tiles_o + o) * groups + y) * 4 + lg) * C + c];
+    ds[idx] += v;
+}
+
 static int tc_wgrad_impl(const float* dy, const float* x, float* dw, const sae_conv_geom* g, cudaStream_t st, const float* mod_s,
                          const float* mod_w, float* mod_ds) {
     if (((reinterpret_cast<uintptr_t>(dy) | reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(dw)) & 15) != 0)
@@ -526,6 +557,9 @@ static int tc_wgrad_impl(const float* dy, const float* x, float* dw, const sae_c
     splits = (p.chunks_total + p.chunks_per_split - 1) / p.chunks_per_split;
 
     if (mod_s != nullptr) p.chunks_per_image = p.tiles_w * p.tiles_h;       // tn == 1 (Q % 32 == 0)
+    p.dw_numel = (int64_t)g->K * p.ntaps * g->C;
+    p.ds_kmax = 0;
+    p.ds_tiles_o = tiles_o;
     static int narrow_mode = -1;
     if (narrow_mode < 0) { const char* v = getenv("SAE_WGRAD_NARROW"); narrow_mode = (v && v[0] == '0') ? 0 : 1; }
     if (mod_s == nullptr && narrow_mode && g->C == 32 && g->stride == 1 && g->S == 3 && g->R <= 3 && p.tw == 32 && g->K <= 128) {
@@ -563,8 +597,12 @@ static int tc_wgrad_impl(const float* dy, const float* x, float* dw, const sae_c
         p.chunks_per_split = (p.chunks_total + nsplit - 1) / nsplit;
         nsplit = (p.chunks_total + p.chunks_per_split - 1) / p.chunks_per_split;
         p.shared_b = 0;
-        wgrad_narrow_kernel<<<(unsigned)nsplit, WG_THREADS, smem_n, st>>>(mdy, mx, dw, p, cols);
-        return check_launch("wgrad_narrow");
+        float* part = det_workspace(det_reduce_floats(p.dw_numel, nsplit));
+        if (!part) return SAE_E_CUDA;
+        wgrad_narrow_kernel<<<(unsigned)nsplit, WG_THREADS, smem_n, st>>>(mdy, mx, part, p, cols);
+        int rc = check_launch("wgrad_narrow");
+        if (rc) return rc;
+        return det_reduce(dw, part, p.dw_numel, nsplit, st);
     }
 
     static int win_mode = -1;
@@ -618,6 +656,21 @@ static int tc_wgrad_impl(const float* dy, const float* x, float* dw, const sae_c
             five_d = 0;
         }
     }
+    // workspace: the per-split partial dW slices (and det_reduce's scratch behind them), then the style-gradient terms
+    const size_t dw_floats = det_reduce_floats(p.dw_numel, splits);
+    size_t ds_floats = 0;
+    if (mod_s != nullptr) {
+        for (int img = 0; img < g->N; ++img) {
+            const int first = (int)(((int64_t)img * p.chunks_per_image) / p.chunks_per_split);
+            const int last = (int)(((int64_t)(img + 1) * p.chunks_per_image - 1) / p.chunks_per_split);
+            if (last - first + 1 > p.ds_kmax) p.ds_kmax = last - first + 1;
+        }
+        ds_floats = (size_t)g->N * p.ds_kmax * tiles_o * groups * 4 * g->C;
+    }
+    float* part = det_workspace(dw_floats + ds_floats);
+    if (!part) return SAE_E_CUDA;
+    if (mod_s != nullptr) p.mod_ds = part + dw_floats;
+    int rc;
     if (pair) {
         constexpr size_t smem = wg_smem_bytes<2>();
         static bool attr_done = false;
@@ -635,18 +688,26 @@ static int tc_wgrad_impl(const float* dy, const float* x, float* dw, const sae_c
         attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
         cfg.attrs = attr;
         cfg.numAttrs = 1;
-        SAE_CUDA_TRY(cudaLaunchKernelEx(&cfg, wgrad_tc_kernel<2>, mdy, mx, dw, p));
-        return check_launch("wgrad_tc<2>");
+        SAE_CUDA_TRY(cudaLaunchKernelEx(&cfg, wgrad_tc_kernel<2>, mdy, mx, part, p));
+        rc = check_launch("wgrad_tc<2>");
+    } else {
+        constexpr size_t smem = wg_smem_bytes<1>();
+        static bool attr_done = false;
+        if (!attr_done) {
+            SAE_CUDA_TRY(cudaFuncSetAttribute(wgrad_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            attr_done = true;
+        }
+        dim3 grid((unsigned)(tiles_o * p.n_tiles_c), (unsigned)groups, (unsigned)splits);
+        wgrad_tc_kernel<1><<<grid, WG_THREADS, smem, st>>>(mdy, mx, part, p);
+        rc = check_launch("wgrad_tc");
     }
-    constexpr size_t smem = wg_smem_bytes<1>();
-    static bool attr_done = false;
-    if (!attr_done) {
-        SAE_CUDA_TRY(cudaFuncSetAttribute(wgrad_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        attr_done = true;
-    }
-    dim3 grid((unsigned)(tiles_o * p.n_tiles_c), (unsigned)groups, (unsigned)splits);
-    wgrad_tc_kernel<1><<<grid, WG_THREADS, smem, st>>>(mdy, mx, dw, p);
-    return check_launch("wgrad_tc");
+    if (rc) return rc;
+    rc = det_reduce(dw, part, p.dw_numel, splits, st);
+    if (rc || mod_s == nullptr) return rc;
+    const int64_t nds = (int64_t)g->N * g->C;
+    mod_ds_reduce_kernel<<<(unsigned)((nds + 255) / 256), 256, 0, st>>>(p.mod_ds, mod_ds, g->N, g->C, p.ds_kmax, tiles_o, groups,
+                                                                      p.chunks_per_image, p.chunks_per_split, splits);
+    return check_launch("mod_ds_reduce");
 }
 
 }  // namespace sae

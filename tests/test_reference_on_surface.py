@@ -1,28 +1,21 @@
-"""CPU, build container only (skipped where /root/reference is absent, e.g. on the GPU box): north_star says the
-reference's ``swapping_autoencoder_model.py`` and ``swapping_autoencoder_optimizer.py`` "consume [the operator surface]
-unchanged".  ``tests/ref_surface_driver.py`` imports the reference's own model / optimizer / network files with
-``models.networks.stylegan2_op`` and ``models.networks.stylegan2_layers`` aliased to this package (INTEGRATION.md §1) and runs
-a D half-step with R1 (double backward) and a G half-step; the same steps through this repo's restated callers
-(model.py / optimizer.py) on the same parameters and seeds must give the same losses and the same updated parameters."""
+"""CPU: north_star says the reference's ``swapping_autoencoder_model.py`` and ``swapping_autoencoder_optimizer.py``
+"consume [the operator surface] unchanged".  ``oracle/ref_surface_driver.py`` imports the reference's own model / optimizer /
+network files with ``models.networks.stylegan2_op`` and ``models.networks.stylegan2_layers`` aliased to this package
+(INTEGRATION.md §1) and runs a D half-step with R1 (double backward) and a G half-step; its losses and updated-parameter
+checksum are stored in ``tests/golden/reference_surface_steps.json`` (``oracle/make_golden.py ref_surface_steps``).  The
+same steps through this repo's restated callers (model.py / optimizer.py) on the same parameters and seeds must give the
+same losses and the same updated parameters."""
 import json
 import math
 import os
-import subprocess
-import sys
 
-import pytest
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get("SAE_REFERENCE_ROOT", "/root/reference")
+from oracle.fixtures import GOLDEN_DIR, surface_steps
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "models", "networks")), reason="reference checkout not present")
-def test_reference_model_and_optimizer_run_on_this_surface():
-    res = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "ref_surface_driver.py"), ROOT, REF],
-                         capture_output=True, text=True, timeout=900, cwd=ROOT)
-    assert res.returncode == 0, res.stdout[-2000:] + res.stderr[-3000:]
-    out = json.loads(res.stdout.strip().splitlines()[-1])
-    ref, ours = out["reference_files"], out["restated_callers"]
+def test_reference_model_and_optimizer_run_on_this_surface(emulated_kernels, fp64_default):
+    import swapping_autoencoder_pytorch_b200 as S
+    ref = json.load(open(os.path.join(GOLDEN_DIR, "reference_surface_steps.json")))["reference_files"]
+    ours = surface_steps(S.create_model, S.create_optimizer)
     for k in ("D/D_real", "D/D_rec", "D/D_mix", "D/PatchD_real", "D/PatchD_mix", "D/D_R1", "D/D_total",
               "G/G_L1", "G/G_GAN_rec", "G/G_GAN_mix", "G/G_mix", "G/L1_dist"):
         assert k in ref and math.isfinite(ref[k]), (k, ref)
