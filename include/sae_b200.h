@@ -31,7 +31,7 @@ extern "C" {
 #define SAE_E_UNSUPPORTED  -3   /* valid request this build has no kernel for                */
 
 /* ABI version of this header; bumped on any signature change. */
-#define SAE_ABI_VERSION 13
+#define SAE_ABI_VERSION 14
 int         sae_abi_version(void);
 const char* sae_last_error(void);
 /* number of kernels launched by this library in the calling process since load
@@ -133,6 +133,32 @@ int sae_modulate(const float* x, const float* s, float* out,
                  int n, int64_t hw, int c, int round_tf32, void* stream);
 int sae_modulate_backward(const float* dy, const float* x, const float* s, float* dx, float* ds,
                           int n, int64_t hw, int c, int round_tf32, void* stream);
+
+/* ------------------------------------------------------------------------------------------
+ * modulate_spatial — the "input * style" step for a spatially varying style (a texture code map
+ * [N, C, h, w], stylegan2_layers.py:269-276 and generator.py:62-67), without the code map ever
+ * reaching the layer's resolution.  The modulation affine commutes with bilinear interpolation
+ * (its weights sum to 1), so the caller evaluates it at the map's own resolution: s_lo [ns, hs, ws, c]
+ * NHWC, ns == 1 (broadcast over the batch) or ns == n.  Per pixel of x [n, h, w, c]:
+ *   v = bilerp(s_lo)(h, w)     F.interpolate(..., size=(h, w), mode='bilinear', align_corners=False):
+ *                              scale = hs / h, src = max(scale (y + 0.5) - 0.5, 0), i0 = floor(src),
+ *                              i1 = i0 + (i0 < hs - 1), lambda = src - i0 (likewise along w)
+ *   u = demodulate ? v * rsqrt(mean_c v^2 + 1e-8) : v
+ *   out = x * u                (rounded to TF32 when round_tf32 != 0)
+ * One read of x and one write of out; any c >= 1 (float4 path when c % 4 == 0 and the pointers are
+ * 16-byte aligned), any ratio between (hs, ws) and (h, w).
+ * backward: dx = dy * u (rounded like the forward) and ds_lo = the adjoint of the interpolation
+ * applied to dv, where g = dy * x and dv = r (g - v r^2 mean_c(g v)), r = rsqrt(mean_c v^2 + 1e-8)
+ * (demodulate) or dv = g; with ns == 1 the adjoint also sums over the batch.  ds_lo is overwritten.
+ * No atomics: a per-pixel pass, then a gather over the columns and one over the rows (and batch) that
+ * each low-resolution cell's stencil touches, in a fixed order — identical inputs give identical bits.
+ * workspace: caller-owned device buffer of 4 * ceil(n * h * ws * c / 4) + 2 * n * h * w floats,
+ * 16-byte aligned.
+ * ------------------------------------------------------------------------------------------ */
+int sae_modulate_spatial(const float* x, const float* s_lo, float* out, int n, int h, int w, int c, int ns, int hs, int ws,
+                         int demodulate, int round_tf32, void* stream);
+int sae_modulate_spatial_backward(const float* dy, const float* x, const float* s_lo, float* dx, float* ds_lo, float* workspace,
+                                  int n, int h, int w, int c, int ns, int hs, int ws, int demodulate, int round_tf32, void* stream);
 
 /* out = (a + b) * scale — the residual merge "(out + skip) / sqrt(2)" of ResBlock (stylegan2_layers.py:691) and of the
  * generator blocks (generator.py:36,53) in one pass; b == NULL gives out = a * scale (its backward).

@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libsae_b200.so")
 CSRC_DIR = os.path.join(_HERE, "csrc")
 
-SAE_ABI_VERSION = 13
+SAE_ABI_VERSION = 14
 
 c_float_p = ctypes.c_void_p   # raw device pointers travel as integers
 c_stream = ctypes.c_void_p
@@ -65,6 +65,8 @@ SIGNATURES = {
                                     ctypes.c_int, c_stream]),
     "sae_modulate_backward": (ctypes.c_int, [c_float_p, c_float_p, c_float_p, c_float_p, c_float_p, ctypes.c_int,
                                              ctypes.c_int64, ctypes.c_int, ctypes.c_int, c_stream]),
+    "sae_modulate_spatial": (ctypes.c_int, [c_float_p] * 3 + [ctypes.c_int] * 9 + [c_stream]),
+    "sae_modulate_spatial_backward": (ctypes.c_int, [c_float_p] * 6 + [ctypes.c_int] * 9 + [c_stream]),
     "sae_add_scale": (ctypes.c_int, [c_float_p, c_float_p, c_float_p, ctypes.c_int64, ctypes.c_float, ctypes.c_int,
                                      c_stream]),
     "sae_round_tf32": (ctypes.c_int, [c_float_p, c_float_p, ctypes.c_int64, c_stream]),

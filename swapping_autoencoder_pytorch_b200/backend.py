@@ -113,6 +113,11 @@ class CudaKernels:
         self.fused_fir_act = os.environ.get("SAE_FUSED_FIR_ACT", "1") != "0"
         # activation bit masks next to the tensor-core convs' / the FIR + activation kernel's outputs (A/B: SAE_ACT_MASK=0)
         self.act_masks = os.environ.get("SAE_ACT_MASK", "1") != "0"
+        # texture code maps [N, C, h, w]: "native" modulates with the affine evaluated at the map's resolution
+        # (sae_modulate_spatial); "glue" interpolates the map to every layer's resolution first (A/B: SAE_SPATIAL_STYLE=glue)
+        self.spatial_style = os.environ.get("SAE_SPATIAL_STYLE", "native")
+        if self.spatial_style not in ("native", "glue"):
+            raise ValueError("SAE_SPATIAL_STYLE must be 'native' or 'glue', not %r" % self.spatial_style)
 
     # ------------------------------------------------------------------ FIR
     def upfirdn2d(self, x, kernel, up_x, up_y, down_x, down_y, pad_x0, pad_x1, pad_y0, pad_y1, taps=None):
@@ -234,6 +239,31 @@ class CudaKernels:
         with torch.cuda.device(x.device):
             check(self.lib.sae_modulate_backward(_ptr(dy), _ptr(x), _ptr(s), _ptr(dx), _ptr(ds), n, h * w, c,
                                                  int(self.round_tf32), _stream()), "sae_modulate_backward")
+        return dx, ds
+
+    def modulate_spatial(self, x, s_lo, demodulate):
+        """x [N,H,W,C] * demod(bilinear(s_lo)) with s_lo [Ns,hs,ws,C], Ns in {1, N} (include/sae_b200.h sae_modulate_spatial)"""
+        _need_cuda(x, s_lo)
+        n, h, w, c = x.shape
+        ns, hs, ws, _ = s_lo.shape
+        out = torch.empty_like(x)
+        with torch.cuda.device(x.device):
+            check(self.lib.sae_modulate_spatial(_ptr(x), _ptr(s_lo), _ptr(out), n, h, w, c, ns, hs, ws, int(demodulate),
+                                                int(self.round_tf32), _stream()), "sae_modulate_spatial")
+        return out
+
+    def modulate_spatial_backward(self, dy, x, s_lo, demodulate):
+        """-> (dx [N,H,W,C], ds_lo [Ns,hs,ws,C])"""
+        _need_cuda(dy, x, s_lo)
+        n, h, w, c = x.shape
+        ns, hs, ws, _ = s_lo.shape
+        dx = torch.empty_like(x)
+        ds = torch.empty_like(s_lo)
+        work = torch.empty((n * h * ws * c + 3) // 4 * 4 + 2 * n * h * w, device=x.device, dtype=x.dtype)
+        with torch.cuda.device(x.device):
+            check(self.lib.sae_modulate_spatial_backward(_ptr(dy), _ptr(x), _ptr(s_lo), _ptr(dx), _ptr(ds), _ptr(work), n, h, w, c, ns,
+                                                         hs, ws, int(demodulate), int(self.round_tf32), _stream()),
+                  "sae_modulate_spatial_backward")
         return dx, ds
 
     # ------------------------------------------------------- residual merge

@@ -1,5 +1,6 @@
 // HBM-bound pointwise kernels: fused bias + (noise) + leaky-relu forward / backward (with the
-// bias-gradient reduction fused in), style modulation forward / backward, gradient bucket
+// bias-gradient reduction fused in), style modulation forward / backward (per sample and, for a
+// texture code map, per pixel), gradient bucket
 // pack / unpack.  Replaces models/networks/stylegan2_op/fused_bias_act_kernel.cu:19-99 and the
 // unfused ATen elementwise kernels listed in SURVEY.md §2.1.
 // All kernels: float4 accesses when the channel count allows, grid = multiple of the SM count,
@@ -247,6 +248,309 @@ modulate_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ x, c
 #pragma unroll
             for (int j = 0; j < VEC; ++j) row[cc * VEC + j] = acc[j];
         }
+    }
+}
+
+// ------------------------------------------------------------------------------ spatially varying modulation
+// A code map modulates every pixel with its own style: u[n,h,w,:] = demod(bilerp(s_lo)(h, w)), where s_lo [Ns, hs, ws, C] is
+// the modulation affine evaluated at the map's own resolution (the affine commutes with bilinear interpolation, whose
+// weights sum to 1).  The interpolation is F.interpolate(..., align_corners=False) for the given output size.
+// Work split: a group of G threads (a power of two <= 32) per pixel; thread gl of the group owns the channel vectors
+// gl, gl + G, ...; the first SP_NV of them (all of them up to C = 512) stay in registers between the two passes a
+// demodulated pixel needs.
+constexpr int SP_NV = 4;
+
+template <int VEC>
+__device__ __forceinline__ void sp_ld(const float* p, float (&r)[VEC]) {
+    if (VEC == 4) {
+        const float4 t = __ldg(reinterpret_cast<const float4*>(p));
+        r[0] = t.x; r[1 % VEC] = t.y; r[2 % VEC] = t.z; r[3 % VEC] = t.w;
+    } else {
+        r[0] = __ldg(p);
+    }
+}
+
+template <int VEC>
+__device__ __forceinline__ void sp_ld_stream(const float* p, float (&r)[VEC]) {
+    if (VEC == 4) {
+        const float4 t = ldg_stream(reinterpret_cast<const float4*>(p));
+        r[0] = t.x; r[1 % VEC] = t.y; r[2 % VEC] = t.z; r[3 % VEC] = t.w;
+    } else {
+        r[0] = p[0];
+    }
+}
+
+template <int VEC>
+__device__ __forceinline__ void sp_st(float* p, const float (&r)[VEC]) {
+    if (VEC == 4) reinterpret_cast<float4*>(p)[0] = make_float4(r[0], r[1 % VEC], r[2 % VEC], r[3 % VEC]);
+    else p[0] = r[0];
+}
+
+// PyTorch's area_pixel_compute_source_index for align_corners=False with scale = in_size / out_size
+__device__ __forceinline__ void sp_src(int d, float scale, int in_size, int& i0, int& i1, float& l0, float& l1) {
+    float src = scale * ((float)d + 0.5f) - 0.5f;
+    if (src < 0.f) src = 0.f;
+    i0 = (int)src;
+    i1 = i0 + (i0 < in_size - 1 ? 1 : 0);
+    l1 = src - (float)i0;
+    l0 = 1.f - l1;
+}
+
+// first output index d in [0, out_size] whose low corner i0(d) is >= k (i0 is non-decreasing in d)
+__device__ __forceinline__ int sp_first_at_least(int k, float scale, int in_size, int out_size) {
+    int d = (int)ceilf(((float)k + 0.5f) / scale - 0.5f);
+    d = d < 0 ? 0 : (d > out_size ? out_size : d);
+    int i0, i1; float l0, l1;
+    while (d > 0) { sp_src(d - 1, scale, in_size, i0, i1, l0, l1); if (i0 < k) break; --d; }
+    while (d < out_size) { sp_src(d, scale, in_size, i0, i1, l0, l1); if (i0 >= k) break; ++d; }
+    return d;
+}
+
+// weight of low-resolution index k in the interpolation stencil of output index d
+__device__ __forceinline__ float sp_weight(int d, int k, float scale, int in_size) {
+    int i0, i1; float l0, l1;
+    sp_src(d, scale, in_size, i0, i1, l0, l1);
+    return (i0 == k ? l0 : 0.f) + (i1 == k ? l1 : 0.f);
+}
+
+struct SpStencil {
+    const float *a, *b, *d, *e;     // corners (y0,x0) (y0,x1) (y1,x0) (y1,x1), channel 0
+    float ly0, ly1, lx0, lx1;
+};
+
+__device__ __forceinline__ SpStencil sp_stencil(const float* s, int64_t n_s, int h, int w, int hs, int ws, int C, float sh, float sw) {
+    SpStencil t;
+    int y0, y1, x0, x1;
+    sp_src(h, sh, hs, y0, y1, t.ly0, t.ly1);
+    sp_src(w, sw, ws, x0, x1, t.lx0, t.lx1);
+    const float* base = s + n_s * hs * ws * C;
+    t.a = base + ((int64_t)y0 * ws + x0) * C; t.b = base + ((int64_t)y0 * ws + x1) * C;
+    t.d = base + ((int64_t)y1 * ws + x0) * C; t.e = base + ((int64_t)y1 * ws + x1) * C;
+    return t;
+}
+
+template <int VEC>
+__device__ __forceinline__ void sp_interp(const SpStencil& t, int c0, float (&v)[VEC]) {
+    float a[VEC], b[VEC], d[VEC], e[VEC];
+    sp_ld<VEC>(t.a + c0, a); sp_ld<VEC>(t.b + c0, b); sp_ld<VEC>(t.d + c0, d); sp_ld<VEC>(t.e + c0, e);
+#pragma unroll
+    for (int j = 0; j < VEC; ++j) v[j] = t.ly0 * (t.lx0 * a[j] + t.lx1 * b[j]) + t.ly1 * (t.lx0 * d[j] + t.lx1 * e[j]);
+}
+
+// out[0:VEC] = a * (v * r), rounded to TF32 when asked
+template <int VEC>
+__device__ __forceinline__ void sp_scale_store(const float (&a)[VEC], const float (&v)[VEC], float r, float* out, int round_tf32) {
+    float y[VEC];
+#pragma unroll
+    for (int j = 0; j < VEC; ++j) {
+        y[j] = a[j] * (v[j] * r);
+        if (round_tf32) y[j] = rna_tf32(y[j]);
+    }
+    sp_st<VEC>(out, y);
+}
+
+__device__ __forceinline__ float sp_group_sum(float v, int G) {
+    for (int o = G >> 1; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+
+// out = x * u, u = bilerp(s_lo) (demodulated per pixel when demod).  The loads of a thread's cached channel vectors are issued
+// before the group reduction, so their HBM latency overlaps it.
+template <int VEC>
+__global__ void __launch_bounds__(256)
+modulate_spatial_kernel(const float* __restrict__ x, const float* __restrict__ s, float* __restrict__ out, int64_t npix, int H, int W,
+                        int C, int bcast, int hs, int ws, float sh, float sw, int G, int demod, int round_tf32) {
+    const int cv = C / VEC;
+    const int lane = threadIdx.x & 31, gl = lane & (G - 1), per_warp = 32 / G;
+    const int64_t warp = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
+    const int64_t step = (((int64_t)gridDim.x * blockDim.x) >> 5) * per_warp;
+    for (int64_t p0 = warp * per_warp; p0 < npix; p0 += step) {         // warp-uniform trip count: every lane reaches the shuffles
+        const int64_t p = p0 + lane / G;
+        const bool valid = p < npix;
+        const int64_t e0 = p * C;
+        SpStencil st;
+        float vc[SP_NV][VEC], xc[SP_NV][VEC];
+        float ss = 0.f;
+        if (valid) {
+            const int64_t n = p / ((int64_t)H * W);
+            const int hw = (int)(p - n * H * W);
+            st = sp_stencil(s, bcast ? 0 : n, hw / W, hw % W, hs, ws, C, sh, sw);
+#pragma unroll
+            for (int k = 0; k < SP_NV; ++k) {
+                const int c = gl + k * G;
+                if (c < cv) {
+                    sp_ld_stream<VEC>(x + e0 + c * VEC, xc[k]);
+                    sp_interp<VEC>(st, c * VEC, vc[k]);
+#pragma unroll
+                    for (int j = 0; j < VEC; ++j) ss = fmaf(vc[k][j], vc[k][j], ss);
+                }
+            }
+            if (demod)
+                for (int c = gl + SP_NV * G; c < cv; c += G) {
+                    float v[VEC];
+                    sp_interp<VEC>(st, c * VEC, v);
+#pragma unroll
+                    for (int j = 0; j < VEC; ++j) ss = fmaf(v[j], v[j], ss);
+                }
+        }
+        float r = 1.f;
+        if (demod) r = rsqrtf(sp_group_sum(ss, G) / (float)C + 1e-8f);
+        if (valid) {
+#pragma unroll
+            for (int k = 0; k < SP_NV; ++k) {
+                const int c = gl + k * G;
+                if (c < cv) sp_scale_store<VEC>(xc[k], vc[k], r, out + e0 + c * VEC, round_tf32);
+            }
+            for (int c = gl + SP_NV * G; c < cv; c += G) {
+                float v[VEC], a[VEC];
+                sp_ld_stream<VEC>(x + e0 + c * VEC, a);
+                sp_interp<VEC>(st, c * VEC, v);
+                sp_scale_store<VEC>(a, v, r, out + e0 + c * VEC, round_tf32);
+            }
+        }
+    }
+}
+
+// backward, per-pixel pass: dx = dy * u and the two per-pixel scalars of the style adjoint, scal[p] = (r, r^2 mean_c(g v)) with
+// g = dy * x, so that dv = r (g - v * scal.y)  (demod) or dv = g (scal = (1, 0))
+template <int VEC>
+__global__ void __launch_bounds__(256)
+modulate_spatial_bwd_pix_kernel(const float* __restrict__ dy, const float* __restrict__ x, const float* __restrict__ s,
+                                float* __restrict__ dx, float2* __restrict__ scal, int64_t npix, int H, int W, int C, int bcast,
+                                int hs, int ws, float sh, float sw, int G, int demod, int round_tf32) {
+    const int cv = C / VEC;
+    const int lane = threadIdx.x & 31, gl = lane & (G - 1), per_warp = 32 / G;
+    const int64_t warp = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
+    const int64_t step = (((int64_t)gridDim.x * blockDim.x) >> 5) * per_warp;
+    for (int64_t p0 = warp * per_warp; p0 < npix; p0 += step) {
+        const int64_t p = p0 + lane / G;
+        const bool valid = p < npix;
+        const int64_t e0 = p * C;
+        SpStencil st;
+        float vc[SP_NV][VEC], gc[SP_NV][VEC];
+        float ss = 0.f, gv = 0.f;
+        if (valid) {
+            const int64_t n = p / ((int64_t)H * W);
+            const int hw = (int)(p - n * H * W);
+            st = sp_stencil(s, bcast ? 0 : n, hw / W, hw % W, hs, ws, C, sh, sw);
+#pragma unroll
+            for (int k = 0; k < SP_NV; ++k) {
+                const int c = gl + k * G;
+                if (c < cv) {
+                    sp_ld_stream<VEC>(dy + e0 + c * VEC, gc[k]);
+                    sp_interp<VEC>(st, c * VEC, vc[k]);
+                    if (demod) {
+                        float xv[VEC];
+                        sp_ld_stream<VEC>(x + e0 + c * VEC, xv);
+#pragma unroll
+                        for (int j = 0; j < VEC; ++j) {
+                            ss = fmaf(vc[k][j], vc[k][j], ss);
+                            gv = fmaf(gc[k][j] * xv[j], vc[k][j], gv);
+                        }
+                    }
+                }
+            }
+            if (demod)
+                for (int c = gl + SP_NV * G; c < cv; c += G) {
+                    float v[VEC], g[VEC], xv[VEC];
+                    sp_interp<VEC>(st, c * VEC, v);
+                    sp_ld_stream<VEC>(dy + e0 + c * VEC, g);
+                    sp_ld_stream<VEC>(x + e0 + c * VEC, xv);
+#pragma unroll
+                    for (int j = 0; j < VEC; ++j) {
+                        ss = fmaf(v[j], v[j], ss);
+                        gv = fmaf(g[j] * xv[j], v[j], gv);
+                    }
+                }
+        }
+        float r = 1.f, a = 0.f;
+        if (demod) {
+            ss = sp_group_sum(ss, G);
+            gv = sp_group_sum(gv, G);
+            r = rsqrtf(ss / (float)C + 1e-8f);
+            a = r * r * gv / (float)C;
+        }
+        if (valid) {
+            if (gl == 0) scal[p] = make_float2(r, a);
+#pragma unroll
+            for (int k = 0; k < SP_NV; ++k) {
+                const int c = gl + k * G;
+                if (c < cv) sp_scale_store<VEC>(gc[k], vc[k], r, dx + e0 + c * VEC, round_tf32);
+            }
+            for (int c = gl + SP_NV * G; c < cv; c += G) {
+                float v[VEC], g[VEC];
+                sp_ld_stream<VEC>(dy + e0 + c * VEC, g);
+                sp_interp<VEC>(st, c * VEC, v);
+                sp_scale_store<VEC>(g, v, r, dx + e0 + c * VEC, round_tf32);
+            }
+        }
+    }
+}
+
+// backward, W-gather: t[n,h,j,:] = sum over the columns w whose stencil touches low-res column j, in order, of wx(w, j) dv[n,h,w,:]
+template <int VEC>
+__global__ void __launch_bounds__(256)
+modulate_spatial_bwd_cols_kernel(const float* __restrict__ dy, const float* __restrict__ x, const float* __restrict__ s,
+                                 const float2* __restrict__ scal, float* __restrict__ t, int64_t total_v, int H, int W, int C,
+                                 int bcast, int hs, int ws, float sh, float sw, int demod) {
+    const int cv = C / VEC;
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total_v; i += (int64_t)gridDim.x * blockDim.x) {
+        const int c0 = (int)(i % cv) * VEC;
+        int64_t q = i / cv;
+        const int j = (int)(q % ws); q /= ws;
+        const int h = (int)(q % H);
+        const int64_t n = q / H;
+        const int w_lo = sp_first_at_least(j - 1, sw, ws, W), w_hi = sp_first_at_least(j + 1, sw, ws, W);
+        float acc[VEC];
+#pragma unroll
+        for (int k = 0; k < VEC; ++k) acc[k] = 0.f;
+        for (int w = w_lo; w < w_hi; ++w) {
+            const float wt = sp_weight(w, j, sw, ws);
+            const int64_t p = (n * H + h) * W + w;
+            float g[VEC], xv[VEC];
+            sp_ld_stream<VEC>(dy + p * C + c0, g);
+            sp_ld_stream<VEC>(x + p * C + c0, xv);
+            if (demod) {
+                const float2 ra = __ldg(scal + p);
+                float v[VEC];
+                sp_interp<VEC>(sp_stencil(s, bcast ? 0 : n, h, w, hs, ws, C, sh, sw), c0, v);
+#pragma unroll
+                for (int k = 0; k < VEC; ++k) acc[k] = fmaf(wt, ra.x * (g[k] * xv[k] - v[k] * ra.y), acc[k]);
+            } else {
+#pragma unroll
+                for (int k = 0; k < VEC; ++k) acc[k] = fmaf(wt, g[k] * xv[k], acc[k]);
+            }
+        }
+        sp_st<VEC>(t + i * VEC, acc);
+    }
+}
+
+// backward, H-gather (and the batch sum of a broadcast map): ds[m,i,j,:] = sum over n, then over the rows h whose stencil
+// touches low-res row i, in order, of wy(h, i) t[n,h,j,:]
+template <int VEC>
+__global__ void __launch_bounds__(256)
+modulate_spatial_bwd_rows_kernel(const float* __restrict__ t, float* __restrict__ ds, int64_t total_v, int N, int H, int C, int bcast,
+                                 int hs, int ws, float sh) {
+    const int cv = C / VEC;
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total_v; i += (int64_t)gridDim.x * blockDim.x) {
+        const int c0 = (int)(i % cv) * VEC;
+        int64_t q = i / cv;
+        const int j = (int)(q % ws); q /= ws;
+        const int r = (int)(q % hs);
+        const int m = (int)(q / hs);
+        const int h_lo = sp_first_at_least(r - 1, sh, hs, H), h_hi = sp_first_at_least(r + 1, sh, hs, H);
+        float acc[VEC];
+#pragma unroll
+        for (int k = 0; k < VEC; ++k) acc[k] = 0.f;
+        for (int n = bcast ? 0 : m; n < (bcast ? N : m + 1); ++n)
+            for (int h = h_lo; h < h_hi; ++h) {
+                const float wt = sp_weight(h, r, sh, hs);
+                float v[VEC];
+                sp_ld<VEC>(t + (((int64_t)n * H + h) * ws + j) * C + c0, v);
+#pragma unroll
+                for (int k = 0; k < VEC; ++k) acc[k] = fmaf(wt, v[k], acc[k]);
+            }
+        sp_st<VEC>(ds + i * VEC, acc);
     }
 }
 
@@ -621,6 +925,75 @@ extern "C" int sae_modulate_backward(const float* dy, const float* x, const floa
     int rc = check_launch("modulate_backward");
     if (rc) return rc;
     return det_reduce(ds, part, (int64_t)n * c, (int)chunks, st);
+}
+
+static int modulate_spatial_check(const char* what, int n, int h, int w, int c, int ns, int hs, int ws) {
+    if (n < 0 || h <= 0 || w <= 0 || c <= 0 || hs <= 0 || ws <= 0 || (ns != 1 && ns != n))
+        return fail(SAE_E_INVALID, "%s: bad sizes (need h, w, c, hs, ws > 0 and ns == 1 or ns == n)", what);
+    return SAE_OK;
+}
+
+// threads per pixel: a power of two <= 32, enough for each to hold at most SP_NV channel vectors where possible (several
+// vectors per thread keep more bytes in flight than one vector per lane)
+static int modulate_spatial_group(int cv) {
+    int g = 1;
+    while (g < 32 && g * SP_NV < cv) g <<= 1;
+    return g;
+}
+
+extern "C" int sae_modulate_spatial(const float* x, const float* s_lo, float* out, int n, int h, int w, int c, int ns, int hs, int ws,
+                                    int demodulate, int round_tf32, void* stream) {
+    if (int rc = modulate_spatial_check("modulate_spatial", n, h, w, c, ns, hs, ws)) return rc;
+    if (n == 0) return SAE_OK;
+    if (!x || !s_lo || !out) return fail(SAE_E_INVALID, "modulate_spatial: null pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    const uintptr_t al = reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(s_lo) | reinterpret_cast<uintptr_t>(out);
+    const int V = (c % 4 == 0 && al % 16 == 0) ? 4 : 1;
+    const int G = modulate_spatial_group(c / V);
+    const int64_t npix = (int64_t)n * h * w;
+    const unsigned blocks = grid_for((npix + 256 / G - 1) / (256 / G) * 256, 256, 16);
+    const float sh = (float)hs / (float)h, sw = (float)ws / (float)w;
+    if (V == 4)
+        modulate_spatial_kernel<4><<<blocks, 256, 0, st>>>(x, s_lo, out, npix, h, w, c, ns == 1, hs, ws, sh, sw, G, demodulate,
+                                                          round_tf32);
+    else
+        modulate_spatial_kernel<1><<<blocks, 256, 0, st>>>(x, s_lo, out, npix, h, w, c, ns == 1, hs, ws, sh, sw, G, demodulate,
+                                                          round_tf32);
+    return check_launch("modulate_spatial");
+}
+
+extern "C" int sae_modulate_spatial_backward(const float* dy, const float* x, const float* s_lo, float* dx, float* ds_lo, float* workspace,
+                                             int n, int h, int w, int c, int ns, int hs, int ws, int demodulate, int round_tf32,
+                                             void* stream) {
+    if (int rc = modulate_spatial_check("modulate_spatial_backward", n, h, w, c, ns, hs, ws)) return rc;
+    if (n == 0) return SAE_OK;
+    if (!dy || !x || !s_lo || !dx || !ds_lo || !workspace) return fail(SAE_E_INVALID, "modulate_spatial_backward: null pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    const uintptr_t al = reinterpret_cast<uintptr_t>(dy) | reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(s_lo) |
+                         reinterpret_cast<uintptr_t>(dx) | reinterpret_cast<uintptr_t>(ds_lo) | reinterpret_cast<uintptr_t>(workspace);
+    const int V = (c % 4 == 0 && al % 16 == 0) ? 4 : 1;
+    const int G = modulate_spatial_group(c / V);
+    const int64_t npix = (int64_t)n * h * w;
+    const int bcast = ns == 1;
+    const float sh = (float)hs / (float)h, sw = (float)ws / (float)w;
+    // workspace: t [n, h, ws, c] (the W-gathered style gradient), then (r, a) per pixel
+    float* t = workspace;
+    float2* scal = reinterpret_cast<float2*>(workspace + ((int64_t)n * h * ws * c + 3) / 4 * 4);
+    const unsigned b_pix = grid_for((npix + 256 / G - 1) / (256 / G) * 256, 256, 16);
+    const int64_t tv_cols = (int64_t)n * h * ws * (c / V), tv_rows = (int64_t)ns * hs * ws * (c / V);
+    if (V == 4) modulate_spatial_bwd_pix_kernel<4><<<b_pix, 256, 0, st>>>(dy, x, s_lo, dx, scal, npix, h, w, c, bcast, hs, ws, sh, sw,
+                                                                           G, demodulate, round_tf32);
+    else        modulate_spatial_bwd_pix_kernel<1><<<b_pix, 256, 0, st>>>(dy, x, s_lo, dx, scal, npix, h, w, c, bcast, hs, ws, sh, sw,
+                                                                           G, demodulate, round_tf32);
+    if (int rc = check_launch("modulate_spatial_backward (pixels)")) return rc;
+    if (V == 4) modulate_spatial_bwd_cols_kernel<4><<<grid_for(tv_cols, 256, 16), 256, 0, st>>>(dy, x, s_lo, scal, t, tv_cols, h, w, c,
+                                                                                                bcast, hs, ws, sh, sw, demodulate);
+    else        modulate_spatial_bwd_cols_kernel<1><<<grid_for(tv_cols, 256, 16), 256, 0, st>>>(dy, x, s_lo, scal, t, tv_cols, h, w, c,
+                                                                                                bcast, hs, ws, sh, sw, demodulate);
+    if (int rc = check_launch("modulate_spatial_backward (columns)")) return rc;
+    if (V == 4) modulate_spatial_bwd_rows_kernel<4><<<grid_for(tv_rows, 256, 16), 256, 0, st>>>(t, ds_lo, tv_rows, n, h, c, bcast, hs, ws, sh);
+    else        modulate_spatial_bwd_rows_kernel<1><<<grid_for(tv_rows, 256, 16), 256, 0, st>>>(t, ds_lo, tv_rows, n, h, c, bcast, hs, ws, sh);
+    return check_launch("modulate_spatial_backward (rows)");
 }
 
 extern "C" int sae_add_scale(const float* a, const float* b, float* out, int64_t n, float scale, int round_tf32, void* stream) {

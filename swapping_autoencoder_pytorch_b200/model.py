@@ -286,6 +286,18 @@ class SwappingAutoencoderModel(BaseModel):
     def decode(self, spatial_code, global_code):
         return self.G(spatial_code, global_code)
 
+    def decode_regions(self, spatial_code, texture_codes, masks):
+        """Region-wise texture editing: decode with texture code k inside region k.  texture_codes [N, K, C]; masks [N, K, hm, wm],
+        non-negative and summing to 1 over K at every pixel (soft masks blend codes).  The code map sum_k masks[:, k] texture_codes[:, k]
+        is built at the masks' resolution and handed to G, which interpolates it to each layer."""
+        if texture_codes.dim() != 3 or masks.dim() != 4 or tuple(masks.shape[:2]) != tuple(texture_codes.shape[:2]):
+            raise ValueError("decode_regions: texture_codes [N, K, C] and masks [N, K, h, w] expected, got %s and %s"
+                             % (tuple(texture_codes.shape), tuple(masks.shape)))
+        if bool((masks < 0).any()) or not torch.allclose(masks.sum(dim=1), masks.new_ones(()), rtol=0.0, atol=1e-4):
+            raise ValueError("decode_regions: masks must be non-negative and sum to 1 over the regions at every pixel")
+        code_map = torch.einsum("nkc,nkhw->nchw", texture_codes, masks.to(texture_codes.dtype))
+        return self.G(spatial_code, code_map)
+
     def get_parameters_for_mode(self, mode):
         if mode == "generator":
             return list(self.G.parameters()) + list(self.E.parameters())

@@ -7,7 +7,7 @@ import torch.nn.functional as F
 
 from .. import util
 from ..stylegan2_layers import ConvLayer, EqualLinear, StyledConv, ToRGB
-from ..stylegan2_op import add_scale, conv2d_residual, upsample2x_add_scale
+from ..stylegan2_op import add_scale, conv2d_residual, spatial_style_native, upsample2x_add_scale
 from .base_network import BaseNetwork
 
 _INV_SQRT2 = 1.0 / math.sqrt(2.0)
@@ -93,7 +93,14 @@ class GeneratorModulation(torch.nn.Module):
     def forward(self, x, style):
         if style.ndimension() <= 2:
             return x * self.scale(style)[:, :, None, None] + self.bias(style)[:, :, None, None]
-        style = F.interpolate(style, size=(x.size(2), x.size(3)), mode='bilinear', align_corners=False)
+        size = (x.size(2), x.size(3))
+        if spatial_style_native():
+            # code map: scale and bias are affine in the code, so they are evaluated at the map's resolution and their
+            # spatial_code_ch-channel results interpolated (exact, bilinear weights sum to 1) — the global_code_ch-channel map
+            # never reaches the structure code's grid
+            return (x * F.interpolate(self.scale(style), size=size, mode='bilinear', align_corners=False)
+                    + F.interpolate(self.bias(style), size=size, mode='bilinear', align_corners=False))
+        style = F.interpolate(style, size=size, mode='bilinear', align_corners=False)
         return x * self.scale(style) + self.bias(style)
 
 

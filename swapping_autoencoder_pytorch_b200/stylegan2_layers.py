@@ -22,7 +22,8 @@ from torch.nn import functional as F
 from .stylegan2_op.blocks import FirSpec, ResBlockSpec, fir_noise_bias_act, fused_blocks_enabled, resblock
 from .stylegan2_op import (FusedLeakyReLU, add_scale, conv2d, conv2d_bias_act, conv2d_noise_bias_act, conv2d_residual,
                            conv_transpose2d, fused_leaky_relu, fused_noise_bias_leaky_relu, linear, memo, modulate,
-                           modulated_conv2d, modulated_conv_ok, reflect_pad, torgb, upfirdn2d)
+                           modulate_spatial, modulated_conv2d, modulated_conv_ok, reflect_pad, spatial_style_native, torgb,
+                           upfirdn2d)
 
 _SQRT2 = math.sqrt(2.0)
 
@@ -236,6 +237,10 @@ class ModulatedConv2d(nn.Module):
         batch = input.shape[0]
         if style.dim() > 2:
             # spatially varying style (reference :269-276; evaluation-time only)
+            if spatial_style_native():
+                # the modulation affine commutes with bilinear interpolation (weights sum to 1): evaluate it at the code map's
+                # resolution and let one kernel interpolate the Cin-channel result, normalise it per pixel and scale the input
+                return modulate_spatial(input, self.modulation(style), self.demodulate)
             style = F.interpolate(style, size=input.shape[2:], mode='bilinear', align_corners=False)
             style = self.modulation(style)
             if self.demodulate:
@@ -380,11 +385,16 @@ class ToRGB(nn.Module):
 
     def forward(self, input, style, skip=None):
         conv = self.conv
-        if (style.dim() <= 2 and not conv.demodulate and conv.kernel_size == 1 and conv.out_channel == 3
-                and not (conv.upsample or conv.downsample) and input.shape[1] % 4 == 0 and input.shape[1] <= 1024):
-            # one pass over the input: style scale, 1x1 conv to 3 channels and bias together (csrc/torgb.cu); no modulated
-            # copy of the generator's largest activation, no N = 3 GEMM
-            s = conv.modulation(style.reshape(input.shape[0], -1))
+        if (not conv.demodulate and conv.kernel_size == 1 and conv.out_channel == 3 and not (conv.upsample or conv.downsample)
+                and input.shape[1] % 4 == 0 and input.shape[1] <= 1024 and (style.dim() <= 2 or spatial_style_native())):
+            # one pass over the input: style scale, 1x1 conv to 3 channels and bias together (csrc/torgb.cu); no N = 3 GEMM and,
+            # for a texture vector, no modulated copy of the generator's largest activation
+            if style.dim() <= 2:
+                s = conv.modulation(style.reshape(input.shape[0], -1))
+            else:
+                # code map: the per-pixel scale is applied first, the kernel then runs with a unit style
+                input = conv.modulated_input(input, style)
+                s = input.new_ones(input.shape[0], input.shape[1])
             out = torgb(input, s, conv.weight[0], self.bias, conv.scale)
         else:
             out = conv(input, style) + self.bias

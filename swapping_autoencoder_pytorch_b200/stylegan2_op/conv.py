@@ -458,6 +458,42 @@ def modulate(x, s):
     return _Modulate.apply(x, s)
 
 
+class _ModulateSpatial(Function):
+    """x * demod(bilinear(s_lo)) for a spatially varying style (stylegan2_layers.py:269-276) whose modulation affine was
+    evaluated at the code map's own resolution: s_lo [Ns, C, hs, ws], Ns in {1, N}.  One pass over x; the style gradient
+    is the interpolation's adjoint, reduced without atomics.  Generator only: once-differentiable."""
+
+    @staticmethod
+    def forward(ctx, x, s_lo, demodulate):
+        xh, sh = _nhwc(x), _nhwc(s_lo)
+        ctx.demodulate = demodulate
+        ctx.save_for_backward(xh, sh)
+        return _nchw(backend.kernels().modulate_spatial(xh, sh, demodulate))
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, dy):
+        xh, sh = ctx.saved_tensors
+        dx, ds = backend.kernels().modulate_spatial_backward(_nhwc(dy), xh, sh, ctx.demodulate)
+        return _nchw(dx), _nchw(ds), None
+
+
+def spatial_style_native():
+    """True when the active kernel set modulates with code maps natively (``modulate_spatial``).  False selects the reference's
+    formulation — interpolate the map to each layer's resolution, then apply the modulation affine there — which
+    ``SAE_SPATIAL_STYLE=glue`` asks of the CUDA kernels and which a kernel set declaring no ``spatial_style`` gets"""
+    return getattr(backend.kernels(), "spatial_style", "glue") == "native"
+
+
+def modulate_spatial(x, s_lo, demodulate):
+    """``x * s`` with ``s = F.interpolate(s_lo, size=x.shape[2:], mode='bilinear', align_corners=False)``, RMS-normalised over
+    channels per pixel when ``demodulate``; s_lo [Ns, C, hs, ws] with Ns == 1 (broadcast) or Ns == x.shape[0]"""
+    n, c = x.shape[:2]
+    if s_lo.dim() != 4 or s_lo.shape[1] != c or s_lo.shape[0] not in (1, n):
+        raise ValueError("modulate_spatial: style map %s does not fit input %s" % (tuple(s_lo.shape), tuple(x.shape)))
+    return _ModulateSpatial.apply(x, s_lo, bool(demodulate))
+
+
 class _ModulatedConv(Function):
     """ModulatedConv2d's core (stylegan2_layers.py:284-323) WITHOUT a modulated copy of the activation: the style scale goes into
     per-sample filters W_n = W * s[n] that the tensor-core kernel selects per pixel tile (``sae_conv2d_fprop_per_sample``),
